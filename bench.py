@@ -2,6 +2,7 @@
 """bench.py — scan-to-map registrations/sec (100k-pt scan vs 1M-pt map) on B200, per BASELINE.json.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload headline|c2|c1|c3|c4|c5]
+                  [--dump-outputs DIR]
 
 One "step" = one NDT registration (pcl::Registration::align semantics) of a synthetic 64-ring scan (~100k points)
 against a 1M-point map, resolution 2.0, DIRECT7, transformation_epsilon 0.01, max 35 iterations, identity guess —
@@ -13,6 +14,9 @@ the steady state apps/align.cpp:32-36 calls "10times" (target already set).
                N_hit*48 + 224) / its CUDA-event duration on the launching stream, vs MEASURED_PEAKS.json hbm_gbs
  * cpu_baseline: the CPU oracle (restatement of the reference's OpenMP path) on the same workload, bounded sample
  * --impl reference: times that CPU path alone (the reference needs PCL/Eigen/FLANN and cannot be built here)
+ * --dump-outputs DIR: after the timed steps, what the timed path returned for each of them (poses, iteration counts, ...)
+               as DIR/<name>.npy; the inputs are seeded, so two builds run with the same arguments compare output for output
+               (to rounding, not bit for bit: the target's voxel moments are summed with f64 atomics in arrival order)
 N > 1: one process per GPU (torchrun), each rank registers its own K scans (replicas — a single alignment does not
 shard, SURVEY.md §8e) and ONE NCCL all-gather of the K 4x4 poses closes the timed region; value = N*K / max time.
 """
@@ -274,6 +278,24 @@ def workload_config(name: str, scans, tgt) -> dict:
                   "stays cache-resident by design (steady-state registration against one map); CPU arm: not applicable"}
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays: dict):
+    """--dump-outputs: every array as <out_dir>/<name>.npy, float32 arrays as they are and all others as float64 (exact for
+    the integer counters and flags). Nothing is written when no directory was given."""
+    if not out_dir:
+        return
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: v if v.dtype == np.float32 else v.astype(np.float64) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed {DUMP_MAX_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v)
+
+
 def make_cpu_ndt(res, threads):
     import oracle
 
@@ -347,12 +369,13 @@ def run_reference(args, rank, world):
     for w in range(args.warmup):
         n.set_source(scans[w % len(scans)])
         n.align()
-    t_total = 0.0
+    t_total, poses = 0.0, []
     for k in range(args.steps):
         n.set_source(scans[k % len(scans)])
         t0 = time.perf_counter()
-        n.align()
+        T = n.align()
         t_total += time.perf_counter() - t0
+        poses.append(T)
     v = args.steps / t_total
     sweep = cpu_thread_sweep(scans, tgt, res, sorted({1, min(8, host_threads())}))
     sweep[str(nt)] = v
@@ -370,6 +393,7 @@ def run_reference(args, rank, world):
         "e2e": {"value": v, "unit": "registrations/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
     print(json.dumps(line), flush=True)
+    dump_outputs(args.dump_outputs, {"pose": np.stack(poses)})
 
 
 def run_c5(args, rank, local_rank, world, m):
@@ -402,15 +426,17 @@ def run_c5(args, rank, local_rank, world, m):
         torch.cuda.synchronize()
         e0.record()
         t0 = time.perf_counter()
-        errs, n_upd, bytes_in = [], 0, 0
+        errs, n_upd, bytes_in, outs = [], 0, 0, []
         for scan, T_gt in frames:
             pose, final, upd = sm.receiveCloud(scan)
             n_upd += int(upd)
             bytes_in += scan.shape[0] * scan.shape[1] * 4
             errs.append(synth.pose_error(final, T_gt)[0])
+            outs.append((pose, final, upd))
         e1.record()
         torch.cuda.synchronize()
         passes.append({"ms": e0.elapsed_time(e1), "wall": time.perf_counter() - t0, "errs": errs, "n_upd": n_upd, "bytes_in": bytes_in,
+                       "outs": outs,
                        "st": sm.stats(), "launches": int(sm.registration.stats()["kernel_launches"] - launches0 + sm.stats()["kernel_launches"])})
     clocks = sampler.stop()
     passes.sort(key=lambda p: p["ms"])
@@ -461,6 +487,8 @@ def run_c5(args, rank, local_rank, world, m):
                          "sample": f"first {n_cpu} frames of the same stream through oracle/scanmatcher.py", "pose_parity_max_m": dpose},
     }
     print(json.dumps(line), flush=True)
+    pose7, final, updated = zip(*mid["outs"])  # per frame of the reported pass: what receiveCloud returned
+    dump_outputs(args.dump_outputs, {"pose7": np.stack(pose7), "final_transformation": np.stack(final), "map_updated": np.array(updated)})
 
 
 def run_c3(args, rank, local_rank, world, m):
@@ -470,7 +498,7 @@ def run_c3(args, rank, local_rank, world, m):
     import torch
 
     base, tgt, res, desc = make_workload("headline", rank)
-    K = min(args.steps, 10)
+    K = args.steps
     scans = step_scans(base, K, rank)
     g = m.GeneralizedIterativeClosestPoint(device=local_rank)
     g.setMaxCorrespondenceDistance(5.0)
@@ -544,6 +572,7 @@ def run_c3(args, rank, local_rank, world, m):
                                           f"{first_cpu:.1f} s on the CPU, {first_s:.2f} s on the GPU)",
                                 "pose_parity": {"dt_m": dt, "dr_rad": dr}, "host": cpu_info()}
     print(json.dumps(line), flush=True)
+    dump_outputs(args.dump_outputs, {"pose": np.stack(poses), "iterations": np.array(its), "evaluations": np.array(evs)})
 
 
 def c4_generate(pairs: int, mine: list[int]):
@@ -572,7 +601,8 @@ def c4_sweep(args, rank, local_rank, world, m, data, with_cpu: bool, comm=None):
     registrations (32-ring scan ~56k pts vs 200k-pt local map, NDT res 2.0, max_iter 100 as graph_based_slam_component.
     cpp:66), the SAME pairs at every N, pair i -> rank i mod N, per pair the node's sequence setInputTarget +
     setInputSource + align + getFitnessScore (gbs.cpp:181, 227-231) from HOST buffers, and ONE all-gather of the result
-    rows INSIDE the timed region. Strong scaling: value = pairs / max-over-ranks time."""
+    rows INSIDE the timed region. Strong scaling: value = pairs / max-over-ranks time. Returns (the line's object, the
+    gathered results) on rank 0 and (None, None) on the other ranks."""
     import torch
     import torch.distributed as dist
 
@@ -606,7 +636,7 @@ def c4_sweep(args, rank, local_rank, world, m, data, with_cpu: bool, comm=None):
     if prev_aff:
         os.sched_setaffinity(0, prev_aff)  # the CPU leg below gets every core back
     if rank != 0:
-        return None
+        return None, None
     errs = [synth.pose_error(res["pose"][k], data[int(i)][2]) for k, i in enumerate(res["index"]) if int(i) in data]
     out = {
         "metric": "loop-closure candidate registrations/sec (64 scan<->submap pairs, sharded)", "value": args.pairs / (ms_max * 1e-3),
@@ -655,7 +685,7 @@ def c4_sweep(args, rank, local_rank, world, m, data, with_cpu: bool, comm=None):
                                    "pose_parity_max": {"dt_m": dmax, "dr_rad": rmax}}
         except Exception as e:  # the GPU numbers must not depend on the CPU leg
             out["cpu_baseline"] = {"value": None, "error": str(e)}
-    return out
+    return out, res
 
 
 def main():
@@ -672,6 +702,8 @@ def main():
     ap.add_argument("--no-flush", action="store_true")
     ap.add_argument("--no-c4", action="store_true", help="skip the loop-closure sweep object of the headline line")
     ap.add_argument("--slots", type=int, default=3, help="registrations in flight per batched launch (1..3)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the timed path returned for each step as DIR/<name>.npy")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -710,11 +742,12 @@ def main():
         sampler = ClockSampler(local_rank)
         sampler.start()
         sampler.arm()
-        c4 = c4_sweep(args, rank, local_rank, world, m, c4_data, with_cpu=False)
+        c4, c4_res = c4_sweep(args, rank, local_rank, world, m, c4_data, with_cpu=False)
         clocks = sampler.stop()
         if rank == 0:
             c4["clocks"] = clocks
             print(json.dumps(c4), flush=True)
+            dump_outputs(args.dump_outputs, c4_res)
         if world > 1:
             dist.destroy_process_group()
         return
@@ -869,9 +902,9 @@ def main():
         all(np.array_equal(rb["pose"][k], re["pose"][k]) and np.array_equal(rb["pose"][k], rp["pose"][k]) for k in range(K))
 
     # ---- the loop-closure sweep (BASELINE config 4) rides in the same line ---------------------------------------
-    c4 = None
+    c4, c4_res = None, None
     if c4_data is not None:
-        c4 = c4_sweep(args, rank, local_rank, world, m, c4_data, with_cpu=not args.no_cpu_baseline, comm=comm)
+        c4, c4_res = c4_sweep(args, rank, local_rank, world, m, c4_data, with_cpu=not args.no_cpu_baseline, comm=comm)
 
     if rank == 0:
         peak, which = hbm_peak()
@@ -940,6 +973,8 @@ def main():
                                     "threads_sweep": sweep, "host": cpu_info(),
                                     "pose_parity_max": {"dt_m": max(e[0] for e in errs), "dr_rad": max(e[1] for e in errs)}}
         print(json.dumps(line), flush=True)
+        # the value leg's batch result (one row per step) and, when it ran, the loop-closure sweep's gathered rows
+        dump_outputs(args.dump_outputs, {**rb, **{"c4_" + k: v for k, v in (c4_res or {}).items()}})
     if world > 1:
         dist.destroy_process_group()
 

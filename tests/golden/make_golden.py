@@ -1,4 +1,6 @@
-"""Generates the committed golden fixtures. Run HERE (the container holding /root/reference), never on the GPU box.
+"""Generates the committed golden fixtures from a checkout of the reference (needs its two vendored scans; no GPU):
+
+    python tests/golden/make_golden.py <path of the lidarslam_ros2 checkout>
 
  * pcd_target_ds.npy / pcd_source_ds.npy: the two vendored scans of the reference
    (Thirdparty/ndt_omp_ros2/data/251370668.pcd = target, 251371071.pcd = source) after the 0.1 m VoxelGrid that
@@ -17,7 +19,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 import oracle  # noqa: E402
 from lidarslam_ros2_b200.pcd import load_pcd  # noqa: E402
 
-REF = "/root/reference/Thirdparty/ndt_omp_ros2/data/"
+REF = os.path.join(sys.argv[1], "Thirdparty", "ndt_omp_ros2", "data", "")
 tgt = load_pcd(REF + "251370668.pcd")
 src = load_pcd(REF + "251371071.pcd")
 tg = oracle.voxelgrid(tgt[:, :3], 0.1)[:, :3].copy()
