@@ -157,8 +157,38 @@ int b200reg_ndt_sweep(b200reg_t h, int count, const float* const* sources, const
 struct b200comm_board;
 int b200reg_ndt_attach_pose_board(b200reg_t h, struct b200comm_board* board);
 int b200reg_ndt_gathered_poses(b200reg_t h, float* poses, int* counts, int max_rows);
-/* registrations in flight per batch launch (1..3; default 3). Developer / measurement switch. */
+/* registrations in flight per batch launch (1..3; default 3; larger values act as 3). Developer / measurement switch.
+ * Any handle kind: b200reg_gicp_align_batch[_device] honours it too. */
 int b200reg_ndt_set_batch_slots(b200reg_t h, int slots);
+
+/* K independent GICP registrations against the handle's CURRENT target in one call — the repeated align() of
+ * apps/align.cpp:32-36 ("10times"), multi-hypothesis initial guesses, or candidate scans sharing one map. Each one runs
+ * computeTransformation (gicp_omp_impl.hpp:369-515) with the handle's parameters; the outer loops advance in lock-step
+ * rounds, and the inner BFGS solves of a round share one persistent launch with up to three of them in flight
+ * (b200reg_ndt_set_batch_slots), so one registration's BFGS arithmetic overlaps the others' cost / gradient sums.
+ * Every result is BITWISE the result b200reg_align gives for the same (source, guess).
+ * guesses: 16*count floats column-major, or NULL (identity). results[k].status is B200REG_OK or an error code
+ * (B200REG_ERR_TIMEOUT: the device watchdog fired during registration k). The target covariances are the handle's
+ * cached ones; the handle's own source and its covariances are not touched (a later align() registers that source as
+ * before). After the call the getters (final transformation, converged, iterations, correspondences) describe the LAST
+ * registration; b200reg_get_stats reports evaluations, gicp_inner_ms, gicp_inner_launches and gicp_pair_evaluations
+ * summed over the batch. count == 0 is a no-op. */
+typedef struct b200reg_gicp_batch_result {
+  float final_T[16];    /* getFinalTransformation(), column-major                          */
+  int converged;        /* hasConverged()                                                   */
+  int iterations;       /* outer iterations (nr_iterations_)                                */
+  int evaluations;      /* cost / gradient evaluations over all inner loops                 */
+  int correspondences;  /* m of the last outer iteration (b200reg_gicp_num_correspondences) */
+  int status, pad;      /* B200REG_OK or an error code                                      */
+} b200reg_gicp_batch_result;
+/* sources in HOST memory: (base, n, stride) clouds as in b200reg_set_input_source, one bulk copy + unpack each, no
+ * synchronisation in between */
+int b200reg_gicp_align_batch(b200reg_t h, int count, const float* const* sources, const size_t* n_points,
+                             size_t stride_bytes, const float* guesses, b200reg_gicp_batch_result* results);
+/* sources already in HBM as float4 (x, y, z, ignored) on the handle's device; read in place (no copy) — they must be
+ * complete when the call is made and stay untouched until it returns */
+int b200reg_gicp_align_batch_device(b200reg_t h, int count, const void* const* dev_sources, const size_t* n_points,
+                                    const float* guesses, b200reg_gicp_batch_result* results);
 
 /* ---- pcl::VoxelGrid<PointXYZI>::filter (sm.cpp:266-269,311-314,325-328,444-447; gbs.cpp:225-226) ------ */
 /* Centroid downsample of all fields (x,y,z,intensity). intensity_offset_bytes < 0: no intensity field.
@@ -178,7 +208,8 @@ typedef struct b200reg_stats {
   int kernel_launches;    /* kernels launched by this handle since creation                              */
   int grid_ctas, block_threads, index_in_smem;
   long long n_voxels, n_cells, n_source, n_target;
-  /* GICP: the persistent inner-loop kernel(s) of the last align (estimateRigidTransformationBFGS on the device)      */
+  /* GICP: the persistent inner-loop kernel(s) of the last align or GICP batch (estimateRigidTransformationBFGS on the
+   * device)                                                                                                          */
   float gicp_inner_ms;             /* their summed device time (CUDA events on the handle's stream)                  */
   int gicp_inner_launches;         /* = outer iterations                                                            */
   double gicp_pair_evaluations;    /* sum over cost / gradient evaluations of the number of correspondences          */

@@ -31,6 +31,7 @@ SYMBOLS = [
     "b200reg_align", "b200reg_get_final_transformation", "b200reg_has_converged",
     "b200reg_get_fitness_score", "b200reg_get_aligned", "b200reg_align_batch",
     "b200reg_ndt_align_batch", "b200reg_ndt_align_batch_device", "b200reg_ndt_set_batch_slots", "b200reg_ndt_sweep",
+    "b200reg_gicp_align_batch", "b200reg_gicp_align_batch_device",
     "b200reg_ndt_attach_pose_board", "b200reg_ndt_gathered_poses",
     "b200reg_voxelgrid", "b200reg_get_stats", "b200reg_ndt_derivatives", "b200reg_ndt_hessian_radius",
     "b200reg_ndt_num_voxels", "b200reg_ndt_get_voxels", "b200reg_nn1",
@@ -60,6 +61,11 @@ class SmStats(C.Structure):
 class BatchResult(C.Structure):
     _fields_ = [("final_T", C.c_float * 16), ("trans_probability", C.c_double), ("converged", C.c_int), ("iterations", C.c_int),
                 ("evaluations", C.c_int), ("status", C.c_int), ("hits_total", C.c_longlong)]
+
+
+class GicpBatchResult(C.Structure):
+    _fields_ = [("final_T", C.c_float * 16), ("converged", C.c_int), ("iterations", C.c_int), ("evaluations", C.c_int),
+                ("correspondences", C.c_int), ("status", C.c_int), ("pad", C.c_int)]
 
 
 class SweepResult(C.Structure):
@@ -132,6 +138,8 @@ def lib() -> C.CDLL:
     L.b200reg_ndt_align_batch.argtypes = [vp, i, vp, vp, sz, vp, vp]
     L.b200reg_ndt_align_batch_device.argtypes = [vp, i, vp, vp, vp, vp]
     L.b200reg_ndt_set_batch_slots.argtypes = [vp, i]
+    L.b200reg_gicp_align_batch.argtypes = [vp, i, vp, vp, sz, vp, vp]
+    L.b200reg_gicp_align_batch_device.argtypes = [vp, i, vp, vp, vp, vp]
     L.b200reg_ndt_attach_pose_board.argtypes = [vp, vp]
     L.b200reg_ndt_gathered_poses.argtypes = [vp, vp, vp, i]
     L.b200reg_ndt_sweep.argtypes = [vp, i, vp, vp, vp, vp, sz, vp, d, vp]

@@ -1143,6 +1143,112 @@ int b200reg_ndt_set_batch_slots(b200reg_t h, int slots) {
 
 }  // extern "C"
 
+// ---- batched GICP registration: K independent scans against the current target, lock-step outer loops ----------------
+namespace {
+// items: device-resident float4 sources + row-major guesses
+int gicp_batch_run(b200reg_t h, int count, const std::vector<GicpBatchItem>& items, b200reg_gicp_batch_result* results) {
+  for (int k = 0; k < count; k++) {  // what a registration that never ran reports
+    std::memset(&results[k], 0, sizeof(results[k]));
+    set_identity(results[k].final_T);
+    results[k].status = B200REG_ERR_NO_TARGET;
+  }
+  if (!h->have_target) return fail(h, B200REG_ERR_NO_TARGET, "gicp_align_batch: no input target");
+  if (count == 0) return B200REG_OK;
+  ensure_nn(h);
+  h->gicp.corr_dist = h->corr_dist;
+  std::vector<GicpBatchOutcome> out((size_t)count);
+  const int slots = std::min(h->batch_slots, GICP_MAX_SLOTS);
+  B200_CUDA(cudaEventRecord(h->ev0, h->stream));
+  h->gicp_solver.align_batch(h->nn, h->d_target.ptr, h->n_target, items.data(), count, h->gicp, slots, h->stream, out.data());
+  B200_CUDA(cudaEventRecord(h->ev1, h->stream));
+  B200_CUDA(cudaEventSynchronize(h->ev1));
+  B200_CUDA(cudaEventElapsedTime(&h->solve_ms, h->ev0, h->ev1));
+  int worst = B200REG_OK;
+  long long evals = 0;
+  for (int k = 0; k < count; k++) {
+    b200reg_gicp_batch_result& r = results[k];
+    const GicpBatchOutcome& o = out[k];
+    if (o.timed_out) {
+      r.status = B200REG_ERR_TIMEOUT;
+      worst = fail(h, B200REG_ERR_TIMEOUT, "GICP batch: the inner-loop kernel watchdog fired");
+      continue;
+    }
+    row_to_col(o.final_T, r.final_T);
+    r.converged = o.converged;
+    r.iterations = o.iterations;
+    r.evaluations = o.evaluations;
+    r.correspondences = o.correspondences;
+    r.status = B200REG_OK;
+    evals += o.evaluations;
+  }
+  // the handle's "last align" state = the last registration of the batch
+  if (count > 0 && results[count - 1].status == B200REG_OK) {
+    std::memcpy(h->final_T, out[count - 1].final_T, sizeof(h->final_T));
+    h->converged = out[count - 1].converged;
+    h->iterations = out[count - 1].iterations;
+  }
+  h->evaluations = (int)evals;
+  return worst;
+}
+}  // namespace
+
+extern "C" {
+
+int b200reg_gicp_align_batch_device(b200reg_t h, int count, const void* const* dev_sources, const size_t* n_points,
+                                    const float* guesses, b200reg_gicp_batch_result* results) {
+  if (!h || h->kind != B200REG_GICP || count < 0 || (count > 0 && (!dev_sources || !n_points || !results))) return B200REG_ERR_ARG;
+  return guarded(h, [&]() {
+    std::vector<GicpBatchItem> items((size_t)count);
+    for (int k = 0; k < count; k++) {
+      if (!dev_sources[k] || n_points[k] == 0) return fail(h, B200REG_ERR_ARG, "gicp_align_batch: empty source cloud");
+      items[k].src = static_cast<const float4*>(dev_sources[k]);
+      items[k].n = n_points[k];
+      if (guesses) col_to_row(guesses + 16 * k, items[k].guess);
+      else set_identity(items[k].guess);
+    }
+    return gicp_batch_run(h, count, items, results);
+  });
+}
+
+int b200reg_gicp_align_batch(b200reg_t h, int count, const float* const* sources, const size_t* n_points, size_t stride_bytes,
+                             const float* guesses, b200reg_gicp_batch_result* results) {
+  if (!h || h->kind != B200REG_GICP || count < 0 || (count > 0 && (!sources || !n_points || !results))) return B200REG_ERR_ARG;
+  if (stride_bytes < 12 || (stride_bytes % 4) != 0) return B200REG_ERR_ARG;
+  return guarded(h, [&]() {
+    size_t total = 0, raw_total = 0;
+    bool pageable = false;
+    std::vector<char> pinned((size_t)count);
+    std::vector<size_t> raw_off((size_t)count);
+    for (int k = 0; k < count; k++) {
+      if (!sources[k] || n_points[k] == 0) return fail(h, B200REG_ERR_ARG, "gicp_align_batch: empty source cloud");
+      total += n_points[k];
+      raw_off[k] = raw_total;
+      raw_total += (n_points[k] * stride_bytes + 255) & ~(size_t)255;
+      pinned[k] = CloudUploader::is_pinned(sources[k]) ? 1 : 0;
+      pageable = pageable || !pinned[k];
+    }
+    if (!h->have_target) return gicp_batch_run(h, count, {}, results);
+    // upload + unpack every source back to back into one device buffer, nothing waits in between
+    h->batch_uploader.reserve(raw_total, pageable);
+    h->d_batch.ensure(total);
+    std::vector<GicpBatchItem> items((size_t)count);
+    size_t off = 0;
+    for (int k = 0; k < count; k++) {
+      h->batch_uploader.upload_at(sources[k], pinned[k] != 0, n_points[k], stride_bytes, -1, 1.0f, h->d_batch.ptr + off, raw_off[k],
+                                  h->stream);
+      items[k].src = h->d_batch.ptr + off;
+      items[k].n = n_points[k];
+      if (guesses) col_to_row(guesses + 16 * k, items[k].guess);
+      else set_identity(items[k].guess);
+      off += n_points[k];
+    }
+    h->other_launches += count;
+    return gicp_batch_run(h, count, items, results);
+  });
+}
+
+}  // extern "C"
+
 // ---- loop-closure candidate sweep on one GPU (generalises gbs.cpp:187-233 from the arg-min candidate to all of them) ----
 namespace {
 int sweep_one(b200reg_t e, const float* src, size_t n_src, const float* tgt, size_t n_tgt, size_t stride, const float* guess,

@@ -84,10 +84,8 @@ __device__ __forceinline__ void inverse3(const double* m, double* o) {
 // One thread per point. The k best (d2, index) pairs are kept in a small unsorted array with the current worst
 // tracked; candidates come from Chebyshev rings of the cell grid until the k-th best distance is inside the
 // searched radius (exact, ties → lower index like the oracle).
-__global__ void __launch_bounds__(128) gicp_cov_kernel(NnView V, const float4* __restrict__ pts, int n, int k, double eps,
-                                                       double* __restrict__ cov6) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
+__device__ __forceinline__ void gicp_cov_point(const NnView& V, const float4* __restrict__ pts, int i, int k, double eps,
+                                               double* __restrict__ cov6) {
   const float4 q = pts[i];
   float bd[GICP_MAX_K];
   int bi[GICP_MAX_K];
@@ -165,6 +163,35 @@ __global__ void __launch_bounds__(128) gicp_cov_kernel(NnView V, const float4* _
   o[3] = 1.0 - w * u[1] * u[1];
   o[4] = -w * u[1] * u[2];
   o[5] = 1.0 - w * u[2] * u[2];
+}
+
+__global__ void __launch_bounds__(128) gicp_cov_kernel(NnView V, const float4* __restrict__ pts, int n, int k, double eps,
+                                                       double* __restrict__ cov6) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  gicp_cov_point(V, pts, i, k, eps, cov6);
+}
+
+}  // namespace
+
+// the clouds of a batched covariance launch: each against its own grid, into its own buffer
+struct GicpCovSource {
+  NnView V;
+  const float4* pts;
+  double* cov6;
+  int n;
+};
+
+namespace {
+
+// K5 over several clouds in one launch (b200reg_gicp_align_batch): blockIdx.y picks the cloud, the points of a cloud are
+// covered exactly as gicp_cov_kernel covers them, so every covariance is bitwise the single path's. (128, 8): 64 registers
+// and no spills with the table entry held in registers.
+__global__ void __launch_bounds__(128, 8) gicp_cov_batch_kernel(const GicpCovSource* __restrict__ sources, int k, double eps) {
+  const GicpCovSource S = sources[blockIdx.y];
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= S.n) return;
+  gicp_cov_point(S.V, S.pts, i, k, eps, S.cov6);
 }
 
 // ---- K6: correspondences + Mahalanobis matrices (gicp_omp_impl.hpp:420-456) ----------------------------------
@@ -368,6 +395,63 @@ void r_derivative(const double* x, const double* R, double* g) {
   g[5] = inner(dPsi);
 }
 
+// ---- outer-loop steps of computeTransformation (:369-515), shared by align() and align_batch() --------------------
+// K6 parameters of one outer iteration: transform_R = transformation_ * guess in f64 (:412-418)
+CorrParams corr_params(const float* transformation, const float* guess16, const GicpConfig& cfg, const double* cov_src,
+                       const double* cov_tgt, size_t n_source) {
+  double TR[16] = {0};
+  for (int i = 0; i < 4; i++)
+    for (int j = 0; j < 4; j++)
+      for (int kk = 0; kk < 4; kk++) TR[i * 4 + j] += double(transformation[i * 4 + kk]) * double(guess16[kk * 4 + j]);
+  CorrParams P;
+  P.cov_src = cov_src;
+  P.cov_tgt = cov_tgt;
+  for (int r = 0; r < 3; r++)
+    for (int c = 0; c < 3; c++) P.R[r * 3 + c] = TR[r * 4 + c];
+  const double dist_threshold = cfg.corr_dist * cfg.corr_dist;
+  P.dist_threshold_d = dist_threshold;
+  P.dist_threshold = dist_threshold > 3.0e38 ? 3.0e38f : (float)dist_threshold;
+  P.n = (int)n_source;
+  return P;
+}
+// the BFGS start: translation and Z-Y-X Euler angles of transformation_ (:198-200)
+void bfgs_start(const float* transformation, double* x) {
+  x[0] = transformation[3];
+  x[1] = transformation[7];
+  x[2] = transformation[11];
+  x[3] = std::atan2(transformation[9], transformation[10]);
+  x[4] = std::asin(-transformation[8]);
+  x[5] = std::atan2(transformation[4], transformation[0]);
+}
+// estimateRigidTransformationBFGS accepts these outcomes and throws on any other (:231-240)
+bool bfgs_accepted(int result, int inner, const GicpConfig& cfg) {
+  return result == BFGS_NoProgress || result == BFGS_Success || inner == cfg.max_inner_iterations;
+}
+// convergence test after outer iteration nr_iterations (:479-505); on convergence previous = transformation
+bool outer_converged(float* previous, const float* transformation, const GicpConfig& cfg, int nr_iterations) {
+  double delta = 0.;
+  for (int a = 0; a < 4; a++)
+    for (int b = 0; b < 4; b++) {
+      const double ratio = (a < 3 && b < 3) ? 1. / cfg.rotation_eps : 1. / cfg.trans_eps;
+      const double cd = ratio * std::fabs(previous[a * 4 + b] - transformation[a * 4 + b]);
+      if (cd > delta) delta = cd;
+    }
+  if (nr_iterations >= cfg.max_iterations || delta < 1) {
+    std::memcpy(previous, transformation, 16 * sizeof(float));
+    return true;
+  }
+  return false;
+}
+// final = previous * guess in f32 (:511)
+void final_transform(const float* previous, const float* guess16, float* out) {
+  for (int i = 0; i < 4; i++)
+    for (int j = 0; j < 4; j++) {
+      float acc = 0;
+      for (int kk = 0; kk < 4; kk++) acc += previous[i * 4 + kk] * guess16[kk * 4 + j];
+      out[i * 4 + j] = acc;
+    }
+}
+
 
 // =====================================================================================================================
 // Persistent inner loop: estimateRigidTransformationBFGS (gicp_omp_impl.hpp:180-241) for one set of correspondences in ONE
@@ -469,7 +553,9 @@ __device__ void r_derivative_dev(const double* x, const double* R, double* g) {
   g[5] = r5;
 }
 
-// the functor the controller CTA's BFGS drives: every thread of the CTA calls it with identical arguments
+// the functor the controller CTA's BFGS drives: every thread of the CTA calls it with identical arguments. It reads the work
+// area (control words + rows), the epoch and m through L: the single launch's own parameters, or those a batched controller
+// fills in for the slot and job it is serving.
 struct GicpDeviceFunctor {
   const GicpInnerLaunch* L;
   double (*red)[K7_SLOTS];  // shared [16][16]
@@ -564,6 +650,122 @@ struct GicpDeviceFunctor {
   }
 };
 
+// estimateRigidTransformationBFGS's inner loop (gicp_omp_impl.hpp:215-230) on the controller CTA; x is updated in place
+__device__ __forceinline__ int gi_minimize(GicpDeviceFunctor& fn, double* x, double gradient_tol, int max_inner, int& inner,
+                                           double& f) {
+  Bfgs6T<GicpDeviceFunctor> bfgs(fn);
+  inner = 0;
+  int result = bfgs.minimizeInit(x);
+  result = BFGS_Running;
+  do {
+    inner++;
+    result = bfgs.minimizeOneStep(x);
+    if (result) break;
+    result = bfgs.testGradient(gradient_tol);
+  } while (result == BFGS_Running && inner < max_inner && !fn.failed);
+  f = bfgs.f;
+  return result;
+}
+
+// the controller tells the evaluators to leave
+__device__ __forceinline__ void gi_publish_exit(GicpInnerWork* W, unsigned seq) {
+  const int tid = threadIdx.x;
+  if (tid < GI_CTL_WORDS) {
+    const unsigned payload = tid == 13 ? (unsigned)GI_MODE_EXIT : 0u;
+    const unsigned long long v = ((unsigned long long)seq << 32) | payload;
+#pragma unroll
+    for (int c = 0; c < GI_CTL_COPIES; c++) gi_st(&W->ctl[c][tid], v);
+  }
+}
+
+__device__ __forceinline__ void gi_write_result(GicpInnerResult* r, const double* x, double f, int status, int inner,
+                                                int evaluations, int failed) {
+  for (int k = 0; k < 6; k++) r->x[k] = x[k];
+  r->f = f;
+  r->status = status;
+  r->inner = inner;
+  r->evaluations = evaluations;
+  r->error = failed ? 1 : 0;
+  __threadfence_system();
+}
+
+// evaluator side of a batched launch: the newest evaluation of a slot whose round is at least `want_round`, as one
+// consistent snapshot of the 14 control words (thread k polls word k) → ctl[], its sequence → seq. Words count when their
+// sequence lies in the launch's block of epochs: seq - base < span (see GicpBatchLaunch). A controller waits only for the
+// evaluators that hold chunks of its job, so an evaluator without one may fall behind by several evaluations and skips
+// them (it has nothing to add to them); an evaluator that holds a chunk blocks its controller and so always sees exactly
+// the evaluation it has to compute. false when the watchdog fired.
+__device__ __forceinline__ bool gi_snapshot_ctl(const unsigned long long* words, unsigned base, unsigned span, unsigned want_round,
+                                                unsigned* ctl, unsigned* seq_sh, int* abort_flag, unsigned* error, unsigned& seq) {
+  const int tid = threadIdx.x;
+  const long long t0 = clock64();
+  for (;;) {
+    if (tid < GI_CTL_WORDS) {
+      unsigned long long v;
+      for (;;) {
+        v = gi_ld(words + tid);
+        const unsigned d = (unsigned)(v >> 32) - base;
+        if (d < span && (d & 0xFFFFu) >= want_round + 1u) break;
+        if (clock64() - t0 > GI_TIMEOUT_CYCLES) {
+          *error = 1;
+          *abort_flag = 1;
+          break;
+        }
+      }
+      ctl[tid] = (unsigned)v;
+      seq_sh[tid] = (unsigned)(v >> 32) - base;
+    }
+    __syncthreads();
+    if (*abort_flag) return false;
+    unsigned newest = seq_sh[0];
+    bool same = true;
+    for (int k = 1; k < GI_CTL_WORDS; k++) {
+      same = same && seq_sh[k] == newest;
+      newest = max(newest, seq_sh[k]);  // a slot's sequences only grow within a launch (its jobs are taken in order)
+    }
+    __syncthreads();  // seq_sh / ctl are rewritten by a retry
+    if (same) {
+      seq = newest;
+      return true;
+    }
+    want_round = (newest & 0xFFFFu) - 1u;  // the controller moved on while the words were read: take the newer evaluation whole
+  }
+}
+
+// evaluator side: the 14 sums of correspondences [i0, i1) by the whole CTA (strided loop, warp shuffles, then the 8 warps
+// in order) published as one row of 16 words. The bits depend only on [i0, i1), not on which CTA computes them.
+__device__ __forceinline__ void gi_chunk_row(const CostParams& P, const float* T, int want_grad, int i0, int i1,
+                                             double (*sm)[K7_SLOTS], double* row) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  double acc[14];
+#pragma unroll
+  for (int k = 0; k < 14; k++) acc[k] = 0.0;
+  for (int i = i0 + tid; i < i1; i += GI_THREADS) cost_point(P, T, want_grad, i, acc);
+#pragma unroll
+  for (int k = 0; k < 14; k++) {
+    double v = acc[k];
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
+    if (lane == 0) sm[warp][k] = v;
+  }
+  __syncthreads();
+  if (tid < K7_SLOTS) {
+    double t = 0;
+    if (tid < 14)
+#pragma unroll
+      for (int w = 0; w < GI_THREADS / 32; w++) t += sm[w][tid];
+    gi_st(reinterpret_cast<unsigned long long*>(row + tid), (unsigned long long)__double_as_longlong(t));
+  }
+  __syncthreads();  // sm (and the caller's ctl) are reused by the next chunk / round
+}
+
+// evaluator CTAs of a launch for a job of n correspondences (the single launch's geometry; the batch keeps it as virtual
+// chunks so that its rows are bitwise the single launch's)
+__host__ __device__ __forceinline__ int gi_eval_chunks(int n, int max_ctas) {
+  const int c = (n + GI_THREADS - 1) / GI_THREADS;
+  return c < max_ctas - 1 ? (c > 1 ? c : 1) : (max_ctas - 1 > 1 ? max_ctas - 1 : 1);
+}
+
 __global__ void __launch_bounds__(GI_THREADS) gicp_inner_kernel(const __grid_constant__ GicpInnerLaunch L) {
   GicpInnerWork* W = L.work;
   const int tid = threadIdx.x;
@@ -656,6 +858,136 @@ __global__ void __launch_bounds__(GI_THREADS) gicp_inner_kernel(const __grid_con
       gi_st(reinterpret_cast<unsigned long long*>(&W->rows[round & 1][rank][tid]), (unsigned long long)__double_as_longlong(t));
     }
     __syncthreads();  // sm and ctl are reused by the next round
+  }
+}
+
+// =====================================================================================================================
+// Batched inner loops (b200reg_gicp_align_batch): the inner solves of one lock-step round of several registrations in ONE
+// cooperative launch. CTAs 0 .. S-1 are controllers, one per slot, each running the BFGS of one job at a time exactly as
+// the single launch's controller does (same functor, own work area); a slot that finishes a job takes the next one from
+// an atomic counter. The other E CTAs are evaluators that serve the slots in turn: wait for slot s's control words (their
+// epoch field names the job), compute the job's virtual chunks e, e + E, ... (the single launch's partition of the job),
+// publish the rows, go on to the next slot. While one slot's controller is in its BFGS arithmetic the evaluators work for
+// the others. A slot takes a further job only while its rounds stay within the 16-bit round field of the sequence words;
+// jobs left untaken go to the next launch.
+// =====================================================================================================================
+constexpr int GI_MAX_ROUNDS = 65534;  // round + 1 must fit below the epoch field of a sequence word
+constexpr int kMaxJobsPerLaunch = 4096;  // the launch's block of epochs (jobs + 1) stays far inside 16 bits
+
+}  // namespace
+
+struct GicpBatchJob {
+  const float4* moved;
+  const int* corr;
+  const float* maha;
+  int n;
+  double x0[6];
+  double m;
+};
+
+namespace {
+
+struct GicpBatchLaunch {
+  const float4* target;
+  const GicpBatchJob* jobs;
+  GicpInnerResult* results;  // pinned host memory, one per job; error stays 3 for a job no slot took
+  GicpInnerWork* work;       // one per slot
+  unsigned* next_job;        // zero at launch
+  int n_jobs, slots, max_ctas;
+  int evals_per_job;         // bound on the evaluations of one job (BFGS line-search limits times max_inner)
+  double gradient_tol;
+  int max_inner;
+  // first of the n_jobs + 1 epochs this launch owns: job j's evaluations carry epoch + j in their sequence words (that is
+  // how the evaluators learn the job), the slots' exit words epoch + n_jobs
+  unsigned epoch;
+};
+
+__global__ void __launch_bounds__(GI_THREADS, 1) gicp_inner_batch_kernel(const __grid_constant__ GicpBatchLaunch L) {
+  const int tid = threadIdx.x;
+  const int S = L.slots;
+  const unsigned seq_base = L.epoch * 65536u;  // sequence of round 0 of job 0
+  if ((int)blockIdx.x < S) {  // ---- controller of slot blockIdx.x ----
+    __shared__ double red[16][K7_SLOTS];
+    __shared__ double tot[K7_SLOTS];
+    __shared__ int job_sh;
+    __shared__ GicpInnerLaunch job_launch;  // what the functor reads: this slot's work area, the epoch, the job's m
+    GicpInnerWork* W = L.work + blockIdx.x;
+    int round = 0, failed = 0;
+    for (;;) {
+      __syncthreads();  // every thread has read the previous job_sh / job_launch
+      if (tid == 0) {
+        int j = -1;
+        if (!failed && (round == 0 || round + L.evals_per_job <= GI_MAX_ROUNDS)) {
+          j = (int)atomicAdd(L.next_job, 1u);
+          if (j >= L.n_jobs) j = -1;
+        }
+        job_sh = j;
+        if (j >= 0) {
+          job_launch.work = W;
+          job_launch.epoch = L.epoch + (unsigned)j;  // the job travels in the epoch field of the sequence words
+          job_launch.m = L.jobs[j].m;
+        }
+      }
+      __syncthreads();
+      const int job = job_sh;
+      if (job < 0) break;
+      const GicpBatchJob& J = L.jobs[job];
+      GicpDeviceFunctor fn{&job_launch, red, tot, gi_eval_chunks(J.n, L.max_ctas), round, 0};
+      double x[6];
+      for (int k = 0; k < 6; k++) x[k] = J.x0[k];
+      int inner;
+      double f;
+      const int result = gi_minimize(fn, x, L.gradient_tol, L.max_inner, inner, f);
+      if (tid == 0) gi_write_result(L.results + job, x, f, result, inner, fn.round - round, fn.failed);
+      round = fn.round;
+      failed = fn.failed;
+    }
+    gi_publish_exit(W, (L.epoch + (unsigned)L.n_jobs) * 65536u + (unsigned)round + 1u);
+    return;
+  }
+  // ---- evaluator CTAs ----
+  __shared__ unsigned ctl[16];
+  __shared__ double sm[GI_THREADS / 32][K7_SLOTS];
+  __shared__ int abort_flag;
+  __shared__ unsigned seq_sh[16];
+  if (tid == 0) abort_flag = 0;
+  const int e = (int)blockIdx.x - S, E = (int)gridDim.x - S;
+  const unsigned span = (unsigned)(L.n_jobs + 1) << 16;  // the jobs' epochs + the exit words' one
+  unsigned long long rounds = 0;  // 16 bits per slot: the slot's next evaluation this CTA expects
+  unsigned live = (1u << S) - 1u;
+  __syncthreads();
+  while (live) {
+    for (int s = 0; s < S; s++) {
+      if (!((live >> s) & 1u)) continue;
+      GicpInnerWork* W = L.work + s;
+      unsigned seq;  // relative to the launch's first epoch: (job << 16) + round + 1
+      if (!gi_snapshot_ctl(&W->ctl[e % GI_CTL_COPIES][0], seq_base, span, (unsigned)(rounds >> (16 * s)) & 0xFFFFu, ctl, seq_sh,
+                           &abort_flag, &W->error, seq))
+        return;
+      const unsigned round = (seq & 0xFFFFu) - 1u;
+      rounds = (rounds & ~(0xFFFFull << (16 * s))) | ((unsigned long long)(round + 1u) << (16 * s));
+      const unsigned mode = ctl[13];
+      float T[12];
+#pragma unroll
+      for (int k = 0; k < 12; k++) T[k] = __uint_as_float(ctl[k]);
+      const int want_grad = (int)ctl[12];
+      __syncthreads();  // ctl is rewritten by the next wait
+      if (mode & (unsigned)GI_MODE_EXIT) {
+        live &= ~(1u << s);
+        continue;
+      }
+      const GicpBatchJob& J = L.jobs[seq >> 16];
+      CostParams P;
+      P.moved = J.moved;
+      P.target = L.target;
+      P.corr = J.corr;
+      P.maha = J.maha;
+      const int n = J.n, n_eval = gi_eval_chunks(n, L.max_ctas), chunk = (n + n_eval - 1) / n_eval;
+      for (int c = e; c < n_eval; c += E) {
+        const int i0 = c * chunk;
+        gi_chunk_row(P, T, want_grad, i0, min(n, i0 + chunk), sm, &W->rows[round & 1][c][0]);
+      }
+    }
   }
 }
 
@@ -814,19 +1146,8 @@ GicpOutcome GicpSolver::align(const NnGrid& target_grid, const float4* target, s
   out.iterations = 0;
   out.evaluations = 0;
   const int k = std::min(cfg.k_correspondences, GICP_MAX_K);
-  if (cov_k_ != k || cov_eps_ != cfg.gicp_epsilon) {
-    target_cov_valid_ = source_cov_valid_ = false;
-    cov_k_ = k;
-    cov_eps_ = cfg.gicp_epsilon;
-  }
   // covariances (lazy, cached per cloud; :381-391). Clouds smaller than k are rejected like :54-58 (left zero).
-  if (!target_cov_valid_) {
-    target_cov_.ensure(n_target * 6 + 6);
-    B200_CUDA(cudaMemsetAsync(target_cov_.ptr, 0, n_target * 6 * sizeof(double), s));
-    if ((size_t)k <= n_target) gicp_covariances(target_grid, target, n_target, k, cfg.gicp_epsilon, target_cov_.ptr, s);
-    target_cov_valid_ = true;
-    launches += 1;
-  }
+  ensure_target_covariances(target_grid, cfg, s);
   if (!source_grid_valid_) {
     source_grid_.build(source, n_source, s);
     source_grid_valid_ = true;
@@ -852,23 +1173,10 @@ GicpOutcome GicpSolver::align(const NnGrid& target_grid, const float4* target, s
   float transformation[16], previous[16];
   set_identity16(transformation);
   set_identity16(previous);
-  const double dist_threshold = cfg.corr_dist * cfg.corr_dist;
   bool converged = false;
   int nr_iterations = 0;
   while (!converged) {
-    // transform_R = transformation_ * guess in f64 (:412-418)
-    double TR[16] = {0};
-    for (int i = 0; i < 4; i++)
-      for (int j = 0; j < 4; j++)
-        for (int kk = 0; kk < 4; kk++) TR[i * 4 + j] += double(transformation[i * 4 + kk]) * double(guess16[kk * 4 + j]);
-    CorrParams P;
-    P.cov_src = source_cov_.ptr;
-    P.cov_tgt = target_cov_.ptr;
-    for (int r = 0; r < 3; r++)
-      for (int c = 0; c < 3; c++) P.R[r * 3 + c] = TR[r * 4 + c];
-    P.dist_threshold_d = dist_threshold;
-    P.dist_threshold = dist_threshold > 3.0e38 ? 3.0e38f : (float)dist_threshold;
-    P.n = (int)n_source;
+    const CorrParams P = corr_params(transformation, guess16, cfg, source_cov_.ptr, target_cov_.ptr, n_source);
     B200_CUDA(cudaMemsetAsync(counter_.ptr, 0, sizeof(unsigned), s));
     // query = transformation_ * output[i] (:426-427); nn1_query applies the 3x4 transform in f32
     nn_idx_.ensure(n_source);
@@ -886,12 +1194,7 @@ GicpOutcome GicpSolver::align(const NnGrid& target_grid, const float4* target, s
 
     // estimateRigidTransformationBFGS (:180-241)
     double x[6];
-    x[0] = transformation[3];
-    x[1] = transformation[7];
-    x[2] = transformation[11];
-    x[3] = std::atan2(transformation[9], transformation[10]);
-    x[4] = std::asin(-transformation[8]);
-    x[5] = std::atan2(transformation[4], transformation[0]);
+    bfgs_start(transformation, x);
     BfgsFunctor6 fn;
     fn.f = [&](const double* xx) {
       float T[16];
@@ -930,30 +1233,13 @@ GicpOutcome GicpSolver::align(const NnGrid& target_grid, const float4* target, s
       } while (result == BFGS_Running && inner < cfg.max_inner_iterations);
     }
     lap(t_inner);
-    if (!(result == BFGS_NoProgress || result == BFGS_Success || inner == cfg.max_inner_iterations)) break;  // throws in the reference
+    if (!bfgs_accepted(result, inner, cfg)) break;  // throws in the reference
     set_identity16(transformation);
     apply_state(transformation, x);
-
-    double delta = 0.;
-    for (int a = 0; a < 4; a++)
-      for (int b = 0; b < 4; b++) {
-        const double ratio = (a < 3 && b < 3) ? 1. / cfg.rotation_eps : 1. / cfg.trans_eps;
-        const double cd = ratio * std::fabs(previous[a * 4 + b] - transformation[a * 4 + b]);
-        if (cd > delta) delta = cd;
-      }
     nr_iterations++;
-    if (nr_iterations >= cfg.max_iterations || delta < 1) {
-      converged = true;
-      std::memcpy(previous, transformation, sizeof(previous));
-    }
+    converged = outer_converged(previous, transformation, cfg, nr_iterations);
   }
-  // final = previous * guess in f32 (:511)
-  for (int i = 0; i < 4; i++)
-    for (int j = 0; j < 4; j++) {
-      float acc = 0;
-      for (int kk = 0; kk < 4; kk++) acc += previous[i * 4 + kk] * guess16[kk * 4 + j];
-      out.final_T[i * 4 + j] = acc;
-    }
+  final_transform(previous, guess16, out.final_T);
   out.converged = converged ? 1 : 0;
   out.iterations = nr_iterations;
   out.evaluations = evaluations_;
@@ -962,6 +1248,239 @@ GicpOutcome GicpSolver::align(const NnGrid& target_grid, const float4* target, s
                          "inner BFGS launches %.3f ms (kernel events %.3f ms), %d outer iterations, %d evaluations\n",
                  t_cov, t_nn, t_inner, inner_ms, nr_iterations, evaluations_);
   return out;
+}
+
+void GicpSolver::ensure_target_covariances(const NnGrid& target_grid, const GicpConfig& cfg, cudaStream_t s) {
+  const int k = std::min(cfg.k_correspondences, GICP_MAX_K);
+  if (cov_k_ != k || cov_eps_ != cfg.gicp_epsilon) {
+    target_cov_valid_ = source_cov_valid_ = false;
+    cov_k_ = k;
+    cov_eps_ = cfg.gicp_epsilon;
+  }
+  if (!target_cov_valid_) {
+    target_cov_.ensure(n_target_ * 6 + 6);
+    B200_CUDA(cudaMemsetAsync(target_cov_.ptr, 0, n_target_ * 6 * sizeof(double), s));
+    if ((size_t)k <= n_target_) gicp_covariances(target_grid, target_, n_target_, k, cfg.gicp_epsilon, target_cov_.ptr, s);
+    target_cov_valid_ = true;
+    launches += 1;
+  }
+}
+
+void GicpSolver::inner_batch_device(int n_jobs, const GicpConfig& cfg, int slots) {
+  const int max_ctas = std::min(sm_count_, GI_MAX_CTAS);
+  if (!d_batch_work_) {
+    B200_CUDA(cudaMalloc(&d_batch_work_, GICP_MAX_SLOTS * sizeof(GicpInnerWork)));
+    B200_CUDA(cudaMemsetAsync(d_batch_work_, 0, GICP_MAX_SLOTS * sizeof(GicpInnerWork), stream_));
+    for (int w = 0; w < GICP_MAX_SLOTS; w++)
+      gi_arm_kernel<<<64, 256, 0, stream_>>>(reinterpret_cast<unsigned long long*>(&d_batch_work_[w].rows[0][0][0]),
+                                            (size_t)2 * GI_MAX_CTAS * K7_SLOTS);
+    B200_CUDA(cudaGetLastError());
+  }
+  if (!ev0_) {
+    B200_CUDA(cudaEventCreate(&ev0_));
+    B200_CUDA(cudaEventCreate(&ev1_));
+  }
+  d_jobs_.ensure((size_t)n_jobs);
+  B200_CUDA(cudaMemcpyAsync(d_jobs_.ptr, h_jobs_.ptr, n_jobs * sizeof(GicpBatchJob), cudaMemcpyHostToDevice, stream_));
+  for (int j = 0; j < n_jobs; j++) h_batch_results_.ptr[j].error = 3;  // "no slot took this job"
+  // a line search evaluates at most 2 * 100 times, plus up to 2 + 2 around it; minimizeInit once
+  const long long per_job = 1 + (long long)std::max(cfg.max_inner_iterations, 1) * (2 * 100 + 4);
+  GicpBatchLaunch L{};
+  L.target = target_;
+  L.work = d_batch_work_;
+  L.next_job = batch_counts_.ptr;
+  L.max_ctas = max_ctas;
+  L.evals_per_job = (int)std::min<long long>(per_job, GI_MAX_ROUNDS + 1);
+  L.gradient_tol = cfg.gradient_tol;
+  L.max_inner = cfg.max_inner_iterations;
+  bool failed = false;
+  for (int first = 0; first < n_jobs && !failed;) {
+    L.jobs = d_jobs_.ptr + first;
+    L.results = h_batch_results_.ptr + first;
+    L.n_jobs = std::min(n_jobs - first, kMaxJobsPerLaunch);
+    L.slots = std::max(1, std::min({slots, L.n_jobs, max_ctas - 1}));
+    L.epoch = inner_epoch_;
+    inner_epoch_ += (unsigned)L.n_jobs + 1u;
+    void* args[] = {&L};
+    {
+      std::lock_guard<std::mutex> coop(cooperative_launch_mutex(device_));
+      // no control word of an earlier launch may pass for one of this launch (whatever the epochs have wrapped to)
+      for (int w = 0; w < L.slots; w++) B200_CUDA(cudaMemsetAsync(&d_batch_work_[w].ctl[0][0], 0, sizeof(d_batch_work_[w].ctl), stream_));
+      B200_CUDA(cudaMemsetAsync(L.next_job, 0, sizeof(unsigned), stream_));
+      B200_CUDA(cudaEventRecord(ev0_, stream_));
+      B200_CUDA(cudaLaunchCooperativeKernel((const void*)gicp_inner_batch_kernel, dim3(max_ctas), dim3(GI_THREADS), args, 0, stream_));
+      B200_CUDA(cudaEventRecord(ev1_, stream_));
+      B200_CUDA(cudaStreamSynchronize(stream_));
+    }
+    launches += 1;
+    float ms = 0;
+    B200_CUDA(cudaEventElapsedTime(&ms, ev0_, ev1_));
+    inner_ms += ms;
+    inner_launches += 1;
+    // the slots take jobs in order from the counter: the solved ones are a prefix
+    const int before = first;
+    while (first < n_jobs && h_batch_results_.ptr[first].error != 3) failed |= h_batch_results_.ptr[first++].error != 0;
+    if (first == before) failed = true;  // no progress: only a launch that never ran leaves every job untaken
+  }
+  if (failed) {  // watchdog: re-arm the rows of every slot and report (the untaken jobs keep error 3)
+    for (int w = 0; w < GICP_MAX_SLOTS; w++) {
+      gi_arm_kernel<<<64, 256, 0, stream_>>>(reinterpret_cast<unsigned long long*>(&d_batch_work_[w].rows[0][0][0]),
+                                            (size_t)2 * GI_MAX_CTAS * K7_SLOTS);
+      B200_CUDA(cudaMemsetAsync(&d_batch_work_[w].error, 0, sizeof(unsigned), stream_));
+    }
+    B200_CUDA(cudaStreamSynchronize(stream_));
+  }
+}
+
+void GicpSolver::align_batch(const NnGrid& target_grid, const float4* target, size_t n_target, const GicpBatchItem* items,
+                             int count, const GicpConfig& cfg, int slots, cudaStream_t s, GicpBatchOutcome* out) {
+  stream_ = s;
+  target_ = target;
+  n_target_ = n_target;
+  evaluations_ = 0;
+  inner_ms = 0;
+  inner_launches = 0;
+  inner_pair_evaluations = 0;
+  ensure_target_covariances(target_grid, cfg, s);
+  if (count <= 0) return;
+  const int k = std::min(cfg.k_correspondences, GICP_MAX_K);
+  while ((int)batch_.size() < count) batch_.emplace_back(new BatchScratch());
+  // source grids and covariances: the grid builds back to back (each reads its cloud's bounds back), then ONE K5 launch
+  // over every cloud of at least k points (smaller ones keep zero covariances, :54-58)
+  h_cov_sources_.ensure((size_t)count);
+  int n_cov = 0;
+  size_t max_n = 0;
+  for (int r = 0; r < count; r++) {
+    BatchScratch& B = *batch_[r];
+    const size_t n = items[r].n;
+    B.grid.build(items[r].src, n, s);
+    B.cov.ensure(n * 6 + 6);
+    B200_CUDA(cudaMemsetAsync(B.cov.ptr, 0, n * 6 * sizeof(double), s));
+    B.maha.ensure(n * 9);
+    B.corr.ensure(n);
+    B.nn_idx.ensure(n);
+    B.nn_d2.ensure(n);
+    B.moved.ensure(n);
+    if ((size_t)k <= n) {
+      h_cov_sources_.ptr[n_cov++] = GicpCovSource{nn_view(B.grid), items[r].src, B.cov.ptr, (int)n};
+      max_n = std::max(max_n, n);
+    }
+  }
+  if (n_cov > 0) {
+    d_cov_sources_.ensure((size_t)n_cov);
+    B200_CUDA(cudaMemcpyAsync(d_cov_sources_.ptr, h_cov_sources_.ptr, n_cov * sizeof(GicpCovSource), cudaMemcpyHostToDevice, s));
+    for (int first = 0; first < n_cov; first += 65535) {  // gridDim.y limit
+      const dim3 grid((unsigned)((max_n + 127) / 128), (unsigned)std::min(65535, n_cov - first));
+      gicp_cov_batch_kernel<<<grid, 128, 0, s>>>(d_cov_sources_.ptr + first, k, cfg.gicp_epsilon);
+      B200_CUDA(cudaGetLastError());
+      launches += 1;
+    }
+  }
+  // "output" = each source transformed by its guess (:397)
+  h_guess12_.ensure((size_t)count * 12);
+  d_guess12_.ensure((size_t)count * 12);
+  for (int r = 0; r < count; r++) std::memcpy(h_guess12_.ptr + 12 * r, items[r].guess, 12 * sizeof(float));
+  B200_CUDA(cudaMemcpyAsync(d_guess12_.ptr, h_guess12_.ptr, count * 12 * sizeof(float), cudaMemcpyHostToDevice, s));
+  for (int r = 0; r < count; r++) {
+    transform_kernel<<<(int)((items[r].n + 255) / 256), 256, 0, s>>>(items[r].src, (int)items[r].n, batch_[r]->moved.ptr,
+                                                                      d_guess12_.ptr + 12 * r);
+    launches += 1;
+  }
+  B200_CUDA(cudaGetLastError());
+
+  // the outer loops in lock-step rounds: round i is outer iteration i of every registration still running
+  struct Reg {
+    float transformation[16], previous[16];
+    bool active = true, converged = false, timed_out = false;
+    int nr_iterations = 0, evaluations = 0, m = 0;
+  };
+  std::vector<Reg> R((size_t)count);
+  for (Reg& g : R) {
+    set_identity16(g.transformation);
+    set_identity16(g.previous);
+  }
+  batch_counts_.ensure((size_t)count + 1);
+  h_batch_counts_.ensure((size_t)count + 1);
+  h_jobs_.ensure((size_t)count);
+  h_batch_results_.ensure((size_t)count);
+  std::vector<int> job_reg;
+  for (;;) {
+    bool any = false;
+    for (const Reg& g : R) any = any || g.active;
+    if (!any) break;
+    // correspondences of every running registration, back to back (stream order keeps the shared grid's query scratch
+    // safe); one read-back of all counts
+    unsigned* counts = batch_counts_.ptr + 1;
+    B200_CUDA(cudaMemsetAsync(counts, 0, count * sizeof(unsigned), s));
+    for (int r = 0; r < count; r++) {
+      if (!R[r].active) continue;
+      BatchScratch& B = *batch_[r];
+      const size_t n = items[r].n;
+      const CorrParams P = corr_params(R[r].transformation, items[r].guess, cfg, B.cov.ptr, target_cov_.ptr, n);
+      nn1_query(target_grid, B.moved.ptr, n, R[r].transformation, B.nn_idx.ptr, B.nn_d2.ptr, s, P.dist_threshold * 1.0001f);
+      gicp_corr_kernel<<<(int)((n + 127) / 128), 128, 0, s>>>(P, B.nn_idx.ptr, B.nn_d2.ptr, B.corr.ptr, B.maha.ptr, counts + r);
+      launches += 1;
+    }
+    B200_CUDA(cudaGetLastError());
+    B200_CUDA(cudaMemcpyAsync(h_batch_counts_.ptr, counts, count * sizeof(unsigned), cudaMemcpyDeviceToHost, s));
+    B200_CUDA(cudaStreamSynchronize(s));
+    // this round's inner solves
+    job_reg.clear();
+    for (int r = 0; r < count; r++) {
+      Reg& g = R[r];
+      if (!g.active) continue;
+      g.m = (int)h_batch_counts_.ptr[r];
+      std::memcpy(g.previous, g.transformation, sizeof(g.previous));
+      if (g.m < 4) {  // NotEnoughPointsException → caught → break (:187-192, :494-498)
+        g.active = false;
+        continue;
+      }
+      GicpBatchJob& J = h_jobs_.ptr[job_reg.size()];
+      J.moved = batch_[r]->moved.ptr;
+      J.corr = batch_[r]->corr.ptr;
+      J.maha = batch_[r]->maha.ptr;
+      J.n = (int)items[r].n;
+      bfgs_start(g.transformation, J.x0);
+      J.m = (double)g.m;
+      job_reg.push_back(r);
+    }
+    if (job_reg.empty()) continue;
+    inner_batch_device((int)job_reg.size(), cfg, slots);
+    for (size_t j = 0; j < job_reg.size(); j++) {
+      Reg& g = R[job_reg[j]];
+      const GicpInnerResult& res = h_batch_results_.ptr[j];
+      if (res.error != 0) {
+        g.timed_out = true;
+        g.active = false;
+        continue;
+      }
+      g.evaluations += res.evaluations;
+      evaluations_ += res.evaluations;
+      inner_pair_evaluations += (double)res.evaluations * (double)g.m;
+      if (!bfgs_accepted(res.status, res.inner, cfg)) {  // throws in the reference
+        g.active = false;
+        continue;
+      }
+      set_identity16(g.transformation);
+      apply_state(g.transformation, res.x);
+      g.nr_iterations++;
+      if (outer_converged(g.previous, g.transformation, cfg, g.nr_iterations)) {
+        g.converged = true;
+        g.active = false;
+      }
+    }
+  }
+  for (int r = 0; r < count; r++) {
+    const Reg& g = R[r];
+    GicpBatchOutcome& o = out[r];
+    final_transform(g.previous, items[r].guess, o.final_T);
+    o.converged = g.converged ? 1 : 0;
+    o.iterations = g.nr_iterations;
+    o.evaluations = g.evaluations;
+    o.correspondences = g.m;
+    o.timed_out = g.timed_out ? 1 : 0;
+  }
+  last_m_ = R[count - 1].m;
 }
 
 }  // namespace b200

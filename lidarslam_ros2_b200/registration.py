@@ -389,6 +389,53 @@ class GeneralizedIterativeClosestPoint(_Registration):
     def setMaximumOptimizerIterations(self, n: int):
         self._check(self._lib.b200reg_gicp_set_maximum_optimizer_iterations(self._h, int(n)))
 
+    # ---- batched registrations against the current target (lock-step outer loops, inner solves share a launch) ----
+    # b200reg_gicp_batch_result as a numpy record
+    _BATCH_DTYPE = np.dtype([("final_T", np.float32, (16,)), ("converged", np.int32), ("iterations", np.int32),
+                             ("evaluations", np.int32), ("correspondences", np.int32), ("status", np.int32), ("pad", np.int32)])
+    _BATCH_FIELDS = ("converged", "iterations", "evaluations", "correspondences", "status")
+
+    def _batch_out(self, res, K):
+        assert self._BATCH_DTYPE.itemsize == C.sizeof(_capi.GicpBatchResult)
+        if K == 0:
+            z = np.zeros(0, dtype=self._BATCH_DTYPE)
+            return {"pose": np.zeros((0, 4, 4), dtype=np.float32), **{k: z[k] for k in self._BATCH_FIELDS}}
+        a = np.frombuffer(res, dtype=self._BATCH_DTYPE, count=K)
+        return {"pose": a["final_T"].reshape(K, 4, 4).transpose(0, 2, 1).copy(),  # column-major -> row-major
+                **{k: a[k].copy() for k in self._BATCH_FIELDS}}
+
+    def alignBatch(self, clouds, guesses=None) -> dict:
+        """K independent align() calls against the current target, sources in HOST memory (b200reg_gicp_align_batch).
+        clouds: list of (N_k, >=3) float32 arrays with equal row stride; guesses: list of 4x4 or None (identity).
+        Each result is bitwise what setInputSource + align(guess) gives; the handle's own source is not touched."""
+        K = len(clouds)
+        cs = [_as_cloud(c) for c in clouds]
+        stride = cs[0].strides[0] if K else 16
+        if any(c.strides[0] != stride for c in cs):
+            raise ValueError("alignBatch: all clouds must share one row stride")
+        ptrs = (C.c_void_p * K)(*[c.ctypes.data for c in cs])
+        ns = (C.c_size_t * K)(*[len(c) for c in cs])
+        g = np.ascontiguousarray(np.stack([_colmajor(x) for x in guesses])) if guesses is not None else None
+        res = (_capi.GicpBatchResult * max(K, 1))()
+        rc = self._lib.b200reg_gicp_align_batch(self._h, K, ptrs, ns, stride, _ptr(g) if g is not None else None, res)
+        self._check(rc, soft=(_capi.ERR_NO_TARGET,))
+        return self._batch_out(res, K)
+
+    def alignBatchDevice(self, dev_ptrs, counts, guesses=None) -> dict:
+        """Same with the sources already in HBM as float4 buffers (b200reg_gicp_align_batch_device), read in place."""
+        K = len(dev_ptrs)
+        ptrs = (C.c_void_p * K)(*[int(p) for p in dev_ptrs])
+        ns = (C.c_size_t * K)(*[int(n) for n in counts])
+        g = np.ascontiguousarray(np.stack([_colmajor(x) for x in guesses])) if guesses is not None else None
+        res = (_capi.GicpBatchResult * max(K, 1))()
+        rc = self._lib.b200reg_gicp_align_batch_device(self._h, K, ptrs, ns, _ptr(g) if g is not None else None, res)
+        self._check(rc, soft=(_capi.ERR_NO_TARGET,))
+        return self._batch_out(res, K)
+
+    def setBatchSlots(self, slots: int):
+        """Registrations in flight per batched inner-loop launch (1..3; larger values act as 3)."""
+        self._check(self._lib.b200reg_ndt_set_batch_slots(self._h, int(slots)))
+
     # ---- parity hooks ----
     def covariances(self, which: str) -> np.ndarray:
         w = 1 if which == "target" else 0
